@@ -11,6 +11,7 @@ workload --config C2 (default, the configuration the metric is quoted on): 3840x
          is cache-resident between steps.  C1/C3/C4/C5 are the other BASELINE.json configs (SURVEY.md 8d).
 
   python bench.py [--config C1..C5] [--gpus N] [--steps K] [--warmup W] [--frames F] [--impl b200|reference]
+                  [--dump-outputs DIR]
 
 Launched under torchrun for N>1 (one rank per GPU): frames are independent units, each rank runs the same
 per-GPU batch (weak scaling) and the encoded byte buffers are gathered to rank 0 over NCCL inside the timed
@@ -219,6 +220,35 @@ def frames_torch(synth, cfg, n, seed0, dev):
     return frames
 
 
+DUMP_MAX_BYTES = 15 << 20        # encoded bytes dumped at most: 60 MiB as float32
+
+
+def dump_outputs(out_dir, out, offs):
+    """What a caller of the batch call receives: the per-frame byte offsets into the output buffer
+    (offsets.npy, float64, all frames) and the encoded bytes (encoded.npy, float32, one value per byte).
+    When all frames' bytes exceed DUMP_MAX_BYTES, encoded.npy holds whole frames taken in a fixed seeded
+    order until the next would not fit (the first frame is cut at the limit if it alone exceeds it), and
+    encoded_frames.npy lists those frames in the order their bytes appear."""
+    os.makedirs(out_dir, exist_ok=True)
+    offs = offs.cpu().numpy().astype(np.int64)
+    np.save(os.path.join(out_dir, "offsets.npy"), offs.astype(np.float64))
+    if offs[-1] <= DUMP_MAX_BYTES:
+        np.save(os.path.join(out_dir, "encoded.npy"), out[:offs[-1]].cpu().numpy().astype(np.float32))
+        return
+    picked, parts, size = [], [], 0
+    for f in np.random.default_rng(SEED).permutation(len(offs) - 1):
+        n = min(int(offs[f + 1] - offs[f]), DUMP_MAX_BYTES - size)
+        if n < offs[f + 1] - offs[f] and picked:
+            break
+        picked.append(int(f))
+        parts.append(out[offs[f]:offs[f] + n].cpu().numpy())
+        size += n
+        if size == DUMP_MAX_BYTES:
+            break
+    np.save(os.path.join(out_dir, "encoded.npy"), np.concatenate(parts).astype(np.float32))
+    np.save(os.path.join(out_dir, "encoded_frames.npy"), np.array(picked, np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -238,7 +268,13 @@ def main():
                     help="N>1: gather through torch.distributed point-to-point (round 1) instead of the C-ABI b200timg_gather")
     ap.add_argument("--exact-scale", action="store_true",
                     help="bit-exact scaler arithmetic on the sixel path instead of the <= 1 LSB fused-multiply-add mode")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's encoded bytes and frame offsets) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl b200)")
     name, cfg = args.config, CONFIGS[args.config]
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -370,6 +406,9 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
     total_bytes = int(offss[0][-1].item())
+    if rank == 0 and args.dump_outputs:        # before the passes below overwrite the output buffers
+        last = (step_no[0] - 1) % nbuf
+        dump_outputs(args.dump_outputs, outs[last], offss[last])
     value = world * F * args.steps * iw * ih / 1e6 / (ms_total / 1e3)
 
     # ---- per-kernel timing (separate pass, profiling on) -> roofline of the dominant kernel

@@ -4,6 +4,8 @@ Every case is (name, dict) where the dict has: frames (list of HxWx4 uint8 array
 one after another to ONE canvas), quarter/upper/color8 flags, x indent in pixels and the
 dy passed for frames after the first (-height = animation / delta mode, 0 = fresh frame).
 """
+import hashlib
+
 import numpy as np
 
 from timg_b200 import synth
@@ -152,6 +154,123 @@ def run_block_case(make_canvas, case):
     for i, fr in enumerate(case["frames"]):
         outs.append(cv.send(fr, case["x"], 0 if i == 0 else case["dy"]))
     return outs
+
+
+def digest(data):
+    """sha256 of an array's or a byte string's bytes: how outputs too large to store are kept as golden data."""
+    if isinstance(data, np.ndarray):
+        data = np.ascontiguousarray(data).tobytes()
+    return hashlib.sha256(data).hexdigest()
+
+
+def random_block_case(seed):
+    """A small random frame and three sparse deltas, random canvas flags."""
+    rng = np.random.default_rng(100 + seed)
+    q, up, c8 = int(rng.integers(0, 2)), int(rng.integers(0, 2)), int(rng.integers(0, 2))
+    w = int(rng.integers(1, 60)) * (2 if q else 1)
+    h = int(rng.integers(1, 50))
+    kind = ["noisea", "photo", "alpha", "noise"][seed % 4]
+    frames = [synth.frame_np(1000 + seed, w, h, kind)]
+    for k in range(3):                      # sparse deltas
+        f = frames[-1].copy()
+        ys, xs = rng.integers(0, h, 5), rng.integers(0, w, 5)
+        f[ys, xs] = rng.integers(0, 256, (5, 4), dtype=np.uint8)
+        frames.append(f)
+    return dict(frames=frames, quarter=q, upper=up, color8=c8, x=int(rng.integers(0, 9)), dy=-h)
+
+
+def random_compose_cases():
+    """(fb, kwargs) for AlphaComposeBackground with random sizes, colours, patterns and start rows."""
+    rng = np.random.default_rng(9)
+    out = []
+    for i in range(10):
+        w, h = int(rng.integers(1, 80)), int(rng.integers(1, 60))
+        fb = synth.frame_np(300 + i, w, h, "noisea")
+        kw = dict(bg=int(rng.integers(0, 2 ** 24)) | 0xff000000, pattern=int(rng.integers(0, 2 ** 32)),
+                  pw=int(rng.integers(0, 5)), ph=int(rng.integers(0, 5)), start_row=int(rng.integers(0, h)))
+        out.append((fb, kw))
+    return out
+
+
+def as256_values():
+    """RGBA words for the 256-colour mapping: random ones plus every threshold of the colour cube and grey ramp."""
+    from timg_b200 import rgba_u32
+    rng = np.random.default_rng(3)
+    vals = list(rng.integers(0, 2 ** 32, 20000, dtype=np.uint64))
+    for r in (0, 46, 47, 48, 114, 115, 154, 155, 194, 195, 234, 235, 255):
+        for g in (0, 47, 115, 255):
+            vals.append(rgba_u32(r, g, r))
+            vals.append(rgba_u32(r, r, r))
+    return [int(v) for v in vals]
+
+
+def random_scale_cases():
+    """(img, ow, oh, fmt) for ImageScaler::Scale: random sizes, arbitrary / integer / one-axis up- and downscales."""
+    rng = np.random.default_rng(2)
+    out = []
+    for it in range(120):
+        iw, ih = int(rng.integers(1, 300)), int(rng.integers(1, 200))
+        mode = it % 5
+        if mode == 0:
+            ow, oh = int(rng.integers(1, 300)), int(rng.integers(1, 200))
+        elif mode == 1:
+            ow, oh = max(1, iw // int(rng.integers(1, 9))), max(1, ih // int(rng.integers(1, 9)))
+        elif mode == 2:
+            ow, oh = iw * int(rng.integers(1, 4)), ih * int(rng.integers(1, 4))
+        elif mode == 3:
+            ow, oh = iw, int(rng.integers(1, 200))
+        else:
+            ow, oh = int(rng.integers(1, 300)), ih
+        img = synth.frame_np(it, iw, ih, ["noisea", "photo", "alpha", "noise"][it % 4])
+        if it % 7 == 0:
+            img[: ih // 2, :, 3] = 0
+        out.append((img, ow, oh, it % 2))
+    return out
+
+
+# ---- BASELINE.json's config geometries, as the GPU tests against the reference's own outputs run them
+CONFIG_GEOMETRIES = [(640, 480, (80, 50, 1, 2, 1.0), "alpha"),            # C1
+                     (3840, 2160, (2700, 1800, 9, 18, 1.0), "photo"),       # C2
+                     (1920, 1080, (320, 100, 2, 2, 2.0), "photo"),          # C3
+                     (3840, 2160, (337, 225, 9, 18, 1.0), "alpha"),         # C4
+                     (1280, 720, (2700, 1800, 9, 18, 1.0), "photo")]       # C5
+CONFIG_BATCH = 64
+
+
+def config_image(iw, ih, kind):
+    return synth.frame_np(11 + iw, iw, ih, kind)
+
+
+def variants(base, n):
+    """n distinct frames from a few generated ones (cheap: a per-frame byte rotation of the colour channels)."""
+    out = np.empty((n,) + base.shape[1:], np.uint8)
+    for f in range(n):
+        fr = base[f % len(base)].copy()
+        fr[..., :3] = fr[..., :3] + np.uint8((37 * (f // len(base))) & 255)
+        out[f] = fr
+    return out
+
+
+def c1_frames():
+    """C1: 64 distinct 640x480 frames (alpha and noise)."""
+    return variants(np.stack([synth.frame_np(500 + i, 640, 480, "alpha" if i % 2 else "noise") for i in range(8)]),
+                    CONFIG_BATCH)
+
+
+def c3_frames():
+    """C3: 64 1080p frames, a photo base with a 64x64 noise sprite moving across it."""
+    iw, ih = 1920, 1080
+    base = synth.frame_np(77, iw, ih, "photo")
+    frames = np.repeat(base[None], CONFIG_BATCH, 0)
+    for k in range(CONFIG_BATCH):
+        x, y = (37 + 8 * k) % (iw - 64), (91 + 5 * k) % (ih - 64)
+        frames[k, y:y + 64, x:x + 64] = synth.frame_np(1077 + k, 64, 64, "noise")
+    return frames
+
+
+def c4_frames():
+    """C4: 64 distinct 4K photo frames."""
+    return variants(np.stack([synth.frame_np(900 + i, 3840, 2160, "photo") for i in range(4)]), CONFIG_BATCH)
 
 
 def scale_cases():

@@ -1,7 +1,6 @@
-"""Pins the CPU oracle (oracle/*.c, our restatement) against
-  (a) the golden fixtures generated from the reference itself (tests/golden/*.npz), always;
-  (b) the reference itself (oracle/_ref/libtimg_ref.so) on fresh random inputs, when built.
-No GPU needed."""
+"""Pins the CPU oracle (oracle/*.c, our restatement) against the golden fixtures generated from the
+reference itself (tests/golden/*.npz, written by tests/golden/make_golden.py): fixed cases and random
+inputs.  No GPU needed."""
 import os
 
 import numpy as np
@@ -9,15 +8,18 @@ import pytest
 
 import cases
 import oracle
-from timg_b200 import synth
 
 G = os.path.join(os.path.dirname(__file__), "golden")
-need_ref = pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (no /root/reference)")
 
 
 @pytest.fixture(scope="module")
 def golden_blocks():
     return np.load(os.path.join(G, "blocks.npz"))
+
+
+@pytest.fixture(scope="module")
+def golden_random():
+    return np.load(os.path.join(G, "reference_random.npz"))
 
 
 @pytest.mark.parametrize("name,case", cases.block_cases(), ids=[n for n, _ in cases.block_cases()])
@@ -66,50 +68,22 @@ def test_config_geometries():
         assert fit(1280, 720, 2700, 1800, 9, 18) == (False, 1280, 720)          # C5 no upscale
 
 
-def test_as256_all_colours():
+def test_as256_all_colours(golden_random):
     import timg_b200
-    rng = np.random.default_rng(3)
-    vals = list(rng.integers(0, 2 ** 32, 20000, dtype=np.uint64))
-    for r in (0, 46, 47, 48, 114, 115, 154, 155, 194, 195, 234, 235, 255):
-        for g in (0, 47, 115, 255):
-            vals.append(oracle.rgba_u32(r, g, r))
-            vals.append(oracle.rgba_u32(r, r, r))
-    want = None
-    if oracle.have_ref():
-        want = [oracle.ref().ref_as256(int(v)) for v in vals]
-    got_o = [oracle.as256(int(v)) for v in vals]
-    got_p = [timg_b200.lib().b200timg_as256(int(v)) for v in vals]
+    vals = cases.as256_values()
+    got_o = [oracle.as256(v) for v in vals]
+    got_p = [timg_b200.lib().b200timg_as256(v) for v in vals]
     assert got_o == got_p
-    if want is not None:
-        assert got_o == want
+    assert got_o == golden_random["as256"].tolist()
 
 
-@need_ref
 @pytest.mark.parametrize("seed", range(6))
-def test_blocks_oracle_vs_reference_random(seed):
-    rng = np.random.default_rng(100 + seed)
-    q, up, c8 = int(rng.integers(0, 2)), int(rng.integers(0, 2)), int(rng.integers(0, 2))
-    w = int(rng.integers(1, 60)) * (2 if q else 1)
-    h = int(rng.integers(1, 50))
-    kind = ["noisea", "photo", "alpha", "noise"][seed % 4]
-    frames = [synth.frame_np(1000 + seed, w, h, kind)]
-    for k in range(3):                      # sparse deltas
-        f = frames[-1].copy()
-        ys, xs = rng.integers(0, h, 5), rng.integers(0, w, 5)
-        f[ys, xs] = rng.integers(0, 256, (5, 4), dtype=np.uint8)
-        frames.append(f)
-    case = dict(frames=frames, quarter=q, upper=up, color8=c8, x=int(rng.integers(0, 9)), dy=-h)
-    a = cases.run_block_case(lambda *f: oracle.BlockCanvas(*f), case)
-    b = cases.run_block_case(lambda *f: oracle.RefBlockCanvas(*f), case)
-    assert a == b
+def test_blocks_oracle_vs_reference_random(seed, golden_random):
+    outs = cases.run_block_case(lambda *f: oracle.BlockCanvas(*f), cases.random_block_case(seed))
+    for i, o in enumerate(outs):
+        assert o == golden_random[f"blocks_{seed}/{i}"].tobytes(), f"frame {i}"
 
 
-@need_ref
-def test_compose_oracle_vs_reference_random():
-    rng = np.random.default_rng(9)
-    for i in range(10):
-        w, h = int(rng.integers(1, 80)), int(rng.integers(1, 60))
-        fb = synth.frame_np(300 + i, w, h, "noisea")
-        kw = dict(bg=int(rng.integers(0, 2 ** 24)) | 0xff000000, pattern=int(rng.integers(0, 2 ** 32)),
-                  pw=int(rng.integers(0, 5)), ph=int(rng.integers(0, 5)), start_row=int(rng.integers(0, h)))
-        assert (oracle.compose_bg(fb, **kw) == oracle.ref_compose_bg(fb, **kw)).all()
+def test_compose_oracle_vs_reference_random(golden_random):
+    for i, (fb, kw) in enumerate(cases.random_compose_cases()):
+        assert (oracle.compose_bg(fb, **kw) == golden_random[f"compose_{i}"]).all(), i

@@ -1,18 +1,27 @@
-"""GPU parity against the REFERENCE ITSELF (oracle/_ref/libtimg_ref.so = the unmodified timg translation units),
-one hop instead of two: the CUDA path is compared with ImageScaler::Scale, Framebuffer::AlphaComposeBackground
-and UnicodeBlockCanvas::Send run in the same test, at the geometries of BASELINE.json's configs, including
-multi-frame batches (>= 64 frames for C3 / C4 / C5) and C3's scaling + delta emission together.
+"""GPU parity against the REFERENCE ITSELF (the unmodified timg translation units), one hop instead of two: the
+CUDA path is compared with what ImageScaler::Scale, Framebuffer::AlphaComposeBackground and UnicodeBlockCanvas::Send
+produced at the geometries of BASELINE.json's configs, including multi-frame batches (>= 64 frames for C3 / C4 /
+C5) and C3's scaling + delta emission together.  Those outputs are too large for the repository, so
+tests/golden/reference_configs.npz keeps their sha256 digests (written by tests/golden/make_golden.py).
 """
+import os
+
 import numpy as np
 import pytest
 
+import cases
 import oracle
 import timg_b200
 from timg_b200 import synth
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref/libtimg_ref.so not built")]
+pytestmark = pytest.mark.gpu
 
 BG = oracle.rgba_u32(0, 0, 0)
+
+
+@pytest.fixture(scope="module")
+def golden():
+    return np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_configs.npz"))
 
 
 def _batch(n, iw, ih, ow, oh, **kw):
@@ -22,79 +31,55 @@ def _batch(n, iw, ih, ow, oh, **kw):
     return timg_b200.Batch(**d)
 
 
-def _variants(base, n):
-    """n distinct frames from a few generated ones (cheap: a per-frame byte rotation of the colour channels)."""
-    out = np.empty((n,) + base.shape[1:], np.uint8)
-    for f in range(n):
-        fr = base[f % len(base)].copy()
-        fr[..., :3] = fr[..., :3] + np.uint8((37 * (f // len(base))) & 255)
-        out[f] = fr
-    return out
-
-
-@pytest.mark.parametrize("iw,ih,fit,kind", [(640, 480, (80, 50, 1, 2, 1.0), "alpha"),            # C1
-                                            (3840, 2160, (2700, 1800, 9, 18, 1.0), "photo"),       # C2
-                                            (1920, 1080, (320, 100, 2, 2, 2.0), "photo"),          # C3
-                                            (3840, 2160, (337, 225, 9, 18, 1.0), "alpha"),         # C4
-                                            (1280, 720, (2700, 1800, 9, 18, 1.0), "photo")])       # C5
-def test_scaler_and_compose_equal_the_reference_at_config_geometries(ctx, iw, ih, fit, kind):
+@pytest.mark.parametrize("iw,ih,fit,kind", cases.CONFIG_GEOMETRIES)
+def test_scaler_and_compose_equal_the_reference_at_config_geometries(ctx, golden, iw, ih, fit, kind):
     _, ow, oh = timg_b200.calc_fit(iw, ih, *fit)
-    img = synth.frame_np(11 + iw, iw, ih, kind)
-    got = ctx.scale(img, ow, oh)
-    want = oracle.ref_scale(img, ow, oh)
-    assert (got == want).all(), int(np.abs(got.astype(int) - want).max())
-    assert (ctx.compose_bg(got, BG) == oracle.ref_compose_bg(want, BG)).all()
+    got = ctx.scale(cases.config_image(iw, ih, kind), ow, oh)
+    assert cases.digest(got) == golden[f"scale_{iw}x{ih}_{ow}x{oh}"]
+    assert cases.digest(ctx.compose_bg(got, BG)) == golden[f"compose_{iw}x{ih}_{ow}x{oh}"]
 
 
-def test_c1_half_blocks_batch_equals_reference_canvas(ctx):
-    n, iw, ih = 64, 640, 480
+def test_c1_half_blocks_batch_equals_reference_canvas(ctx, golden):
+    n, iw, ih = cases.CONFIG_BATCH, 640, 480
     _, ow, oh = timg_b200.calc_fit(iw, ih, 80, 50, 1, 2)
-    frames = _variants(np.stack([synth.frame_np(500 + i, iw, ih, "alpha" if i % 2 else "noise") for i in range(8)]), n)
-    outs = ctx.blocks_batch(frames, _batch(n, iw, ih, ow, oh))
+    outs = ctx.blocks_batch(cases.c1_frames(), _batch(n, iw, ih, ow, oh))
     for f in range(n):
-        fb = oracle.ref_compose_bg(oracle.ref_scale(frames[f], ow, oh), BG)
-        assert outs[f] == oracle.RefBlockCanvas(False).send(fb), f
+        assert cases.digest(outs[f]) == golden["c1_half"][f], f
 
 
-def test_c3_quarter_animation_scale_plus_delta_equals_reference_canvas(ctx):
+def test_c3_quarter_animation_scale_plus_delta_equals_reference_canvas(ctx, golden):
     """C3: 1080p -> 320x90 -> -p quarter, 64 frames, frame 0 full and the rest emitted as differences, scaling and
     delta emission in ONE batch call, against the reference's scaler + compose + ONE stateful UnicodeBlockCanvas."""
-    n, iw, ih = 64, 1920, 1080
+    n, iw, ih = cases.CONFIG_BATCH, 1920, 1080
     _, ow, oh = timg_b200.calc_fit(iw, ih, 320, 100, 2, 2, 2.0)
     assert (ow, oh) == (320, 90)
-    base = synth.frame_np(77, iw, ih, "photo")
-    frames = np.repeat(base[None], n, 0)
-    for k in range(n):
-        x, y = (37 + 8 * k) % (iw - 64), (91 + 5 * k) % (ih - 64)
-        frames[k, y:y + 64, x:x + 64] = synth.frame_np(1077 + k, 64, 64, "noise")
-    outs = ctx.blocks_batch(frames, _batch(n, iw, ih, ow, oh, flags=timg_b200.QUARTER, animation=1))
-    cv = oracle.RefBlockCanvas(True)
+    outs = ctx.blocks_batch(cases.c3_frames(), _batch(n, iw, ih, ow, oh, flags=timg_b200.QUARTER, animation=1))
     for f in range(n):
-        fb = oracle.ref_compose_bg(oracle.ref_scale(frames[f], ow, oh), BG)
-        want = cv.send(fb, 0, 0 if f == 0 else -oh)
         prefix = b"" if f == 0 else b"\033[%dA" % (oh // 2)      # the adapter adds the cursor-up, the ABI returns image bytes
-        assert prefix + outs[f] == want, f
+        assert cases.digest(prefix + outs[f]) == golden["c3_quarter_delta"][f], f
     assert sum(len(o) for o in outs[1:]) < len(outs[0]) * (n - 1) // 4      # deltas really are deltas
 
 
-def test_c4_grid_sixel_batch_of_64_equals_staged_reference_scaler(ctx):
+def test_c4_grid_sixel_batch_of_64_equals_staged_reference_scaler(ctx, golden):
     """C4: 64 distinct 4K frames -> 337x190 (+pad 192) sixel in one batch == reference scaler + compose per frame,
-    then the single-frame encoder (whose own parity is covered in test_sixel_gpu.py)."""
-    n, iw, ih = 64, 3840, 2160
+    then the single-frame encoder (whose own parity is covered in test_sixel_gpu.py).  The staged frames are
+    rebuilt with the CPU restatements and must hash to the reference's own."""
+    n, iw, ih = cases.CONFIG_BATCH, 3840, 2160
     _, ow, oh = timg_b200.calc_fit(iw, ih, 337, 225, 9, 18)
-    frames = _variants(np.stack([synth.frame_np(900 + i, iw, ih, "photo") for i in range(4)]), n)
+    frames = cases.c4_frames()
     outs = ctx.sixel_batch(frames, _batch(n, iw, ih, ow, oh))
     hp = (oh + 5) // 6 * 6
     for f in range(n):
         fb = np.zeros((hp, ow, 4), np.uint8)
-        fb[:oh] = oracle.ref_compose_bg(oracle.ref_scale(frames[f], ow, oh), BG)
-        fb = oracle.ref_compose_bg(fb, BG, start_row=oh)                    # SixelCanvas::Send's pad strip
+        fb[:oh] = oracle.compose_bg(oracle.stb_resize(frames[f], ow, oh), BG)
+        fb = oracle.compose_bg(fb, BG, start_row=oh)                        # SixelCanvas::Send's pad strip
+        assert cases.digest(fb) == golden["c4_staged"][f], f
         assert outs[f] == ctx.sixel_encode(fb), f
 
 
 def test_c5_unscaled_720p_sixel_batch_of_64(ctx):
     n, w, h = 64, 1280, 720
-    frames = _variants(np.stack([synth.frame_np(200 + i, w, h, "photo") for i in range(8)]), n)
+    frames = cases.variants(np.stack([synth.frame_np(200 + i, w, h, "photo") for i in range(8)]), n)
     outs = ctx.sixel_batch(frames, _batch(n, w, h, w, h))
     for f in range(0, n, 7):                                               # every 7th frame against the CPU restatement (0.1 s each)
         img, used = oracle.sixel_decode(outs[f])

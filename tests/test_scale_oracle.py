@@ -4,15 +4,12 @@ oracle's.  No GPU needed."""
 import os
 
 import numpy as np
-import pytest
 
 import cases
 import oracle
 import timg_b200
-from timg_b200 import synth
 
 G = os.path.join(os.path.dirname(__file__), "golden")
-need_ref = pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built")
 
 
 def test_scale_oracle_matches_golden():
@@ -69,24 +66,8 @@ def test_c2_plan_shape():
     np.testing.assert_allclose(v["coeff"].sum(1), 1.0, atol=1e-6)
 
 
-@need_ref
 def test_scale_oracle_vs_reference_random():
-    rng = np.random.default_rng(2)
-    for it in range(120):
-        iw, ih = int(rng.integers(1, 300)), int(rng.integers(1, 200))
-        mode = it % 5
-        if mode == 0:
-            ow, oh = int(rng.integers(1, 300)), int(rng.integers(1, 200))
-        elif mode == 1:
-            ow, oh = max(1, iw // int(rng.integers(1, 9))), max(1, ih // int(rng.integers(1, 9)))
-        elif mode == 2:
-            ow, oh = iw * int(rng.integers(1, 4)), ih * int(rng.integers(1, 4))
-        elif mode == 3:
-            ow, oh = iw, int(rng.integers(1, 200))
-        else:
-            ow, oh = int(rng.integers(1, 300)), ih
-        img = synth.frame_np(it, iw, ih, ["noisea", "photo", "alpha", "noise"][it % 4])
-        if it % 7 == 0:
-            img[: ih // 2, :, 3] = 0
-        fmt = it % 2
-        assert (oracle.stb_resize(img, ow, oh, fmt) == oracle.ref_scale(img, ow, oh, fmt)).all(), (iw, ih, ow, oh)
+    """The reference's outputs on these inputs are stored as digests (they would not fit the repository)."""
+    want = np.load(os.path.join(G, "reference_random.npz"))["scale"]
+    for (img, ow, oh, fmt), d in zip(cases.random_scale_cases(), want, strict=True):
+        assert cases.digest(oracle.stb_resize(img, ow, oh, fmt)) == d, (img.shape, ow, oh, fmt)
