@@ -85,6 +85,11 @@ ABI = {
     "b200timg_base64_size": (C.c_size_t, [C.c_size_t]),
     "b200timg_png_encode": (C.c_int, [C.c_void_p, u8p, C.c_int, C.c_int, C.c_int, u8p, C.c_size_t, C.c_char_p, C.c_size_t]),
     "b200timg_png_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "b200timg_png_bound": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "b200timg_png_encode_level": (C.c_int, [C.c_void_p, u8p, C.c_int, C.c_int, C.c_int, C.c_int, u8p, C.c_size_t,
+                                            C.POINTER(C.c_size_t), C.c_char_p, C.c_size_t]),
+    "b200timg_png_batch_level_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                               C.c_size_t, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200timg_gather_unique_id": (C.c_int, [C.c_char_p]),
     "b200timg_gather_init": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.c_int]),
     "b200timg_gather_attach": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int]),
@@ -231,16 +236,27 @@ class Context:
         self._chk(lib().b200timg_windows(self.h, _np_ptr(img), w, h, dw, dh, x0, y0, dx, dy, first_pos, n_pos, _np_ptr(out)))
         return out
 
-    def png_encode(self, fb, rgb24=False, want_base64=True):
-        """(PNG bytes, base64 text or None) of an RGBA frame, as the kitty / iTerm2 canvases would send it."""
+    def png_encode(self, fb, rgb24=False, want_base64=True, level=0):
+        """(PNG bytes, base64 text or None) of an RGBA frame, as the kitty / iTerm2 canvases would send it.
+        level: timg's --compress (0 stored blocks, 1..9 deflate-compressed)."""
         fb = np.ascontiguousarray(fb, dtype=np.uint8)
         h, w = fb.shape[:2]
-        n = lib().b200timg_png_size(w, h, int(rgb24))
-        out = np.empty(n, np.uint8)
-        nb = lib().b200timg_base64_size(n)
+        if level == 0:
+            n = lib().b200timg_png_size(w, h, int(rgb24))
+            out = np.empty(n, np.uint8)
+            nb = lib().b200timg_base64_size(n)
+            b64 = C.create_string_buffer(nb) if want_base64 else None
+            self._chk(lib().b200timg_png_encode(self.h, _np_ptr(fb), w, h, int(rgb24), _np_ptr(out), n, b64, nb if want_base64 else 0))
+            return out.tobytes(), (b64.raw if want_base64 else None)
+        cap = lib().b200timg_png_bound(w, h, int(rgb24), level)
+        out = np.empty(cap, np.uint8)
+        nb = lib().b200timg_base64_size(cap)
         b64 = C.create_string_buffer(nb) if want_base64 else None
-        self._chk(lib().b200timg_png_encode(self.h, _np_ptr(fb), w, h, int(rgb24), _np_ptr(out), n, b64, nb if want_base64 else 0))
-        return out.tobytes(), (b64.raw if want_base64 else None)
+        n = C.c_size_t()
+        self._chk(lib().b200timg_png_encode_level(self.h, _np_ptr(fb), w, h, int(rgb24), level, _np_ptr(out), cap, C.byref(n),
+                                                  b64, nb if want_base64 else 0))
+        data = out[:n.value].tobytes()
+        return data, (b64.raw[:lib().b200timg_base64_size(n.value)] if want_base64 else None)
 
     def compose_bg(self, fb, bg, pattern=0, pw=0, ph=0, start_row=0, has_bg=True):
         out = np.ascontiguousarray(fb, dtype=np.uint8).copy()

@@ -73,7 +73,7 @@ void b200timg_ctx_destroy(b200timg_ctx *ctx) {
     ctx->gather_status.release();
     ctx->in_stage.release(); ctx->fb_scaled.release(); ctx->prev_stage.release();
     ctx->out_stage.release(); ctx->offsets.release(); ctx->cells.release(); ctx->rows.release();
-    ctx->tables.release(); ctx->sixel_work.release(); ctx->misc.release(); ctx->scale_list.release(); ctx->scale_tmp.release(); ctx->tri_tables.release();
+    ctx->tables.release(); ctx->sixel_work.release(); ctx->misc.release(); ctx->deflate_work.release(); ctx->scale_list.release(); ctx->scale_tmp.release(); ctx->tri_tables.release();
     ctx->pinned.release(); ctx->pinned_io.release();
     for (int i = 0; i < 2; ++i) { ctx->pipe_in[i].release(); ctx->pipe_out[i].release(); }
     if (ctx->parts_ready) {

@@ -81,6 +81,7 @@ struct b200timg_ctx {
     b200timg::DevBuf tables;       // resampler coefficient tables
     b200timg::DevBuf sixel_work;   // palettes, LUTs, index planes, band tables
     b200timg::DevBuf misc;         // small flags / sizes
+    b200timg::DevBuf deflate_work; // compressed PNG: per-segment output slots, sizes and offsets (deflate.cu)
     b200timg::DevBuf tri_tables;   // bilinear / YUV scaler tap tables ...
     int tri_key[5] = {0, 0, 0, 0, 0};          // ... for this (kind, iw, ih, ow, oh), device pointers cached in tri_params
     std::vector<char> tri_params;
